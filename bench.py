@@ -92,7 +92,31 @@ def parse_args():
     p.add_argument("--profile-steps", type=int, default=20, help="reverse steps of the CUDA-event kernel profile")
     p.add_argument("--no-extra-workloads", action="store_true", help="skip the short config 3 / config 5 sub-lines")
     p.add_argument("--no-parity", action="store_true", help="skip the parity block")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """
+    Write each array as DIR/<name>.npy in float32, so that two builds run with the same arguments (hence the same
+    seeded inputs) can be compared output for output.  Where the arrays together exceed 64 MB, each keeps a fixed,
+    seeded sample of its rows (leading axis), the same for every build.
+    """
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, a.shape[0] * DUMP_LIMIT_BYTES // total)
+            a = a[np.sort(np.random.default_rng(SEED).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
 
 
 def workload(args):
@@ -326,6 +350,8 @@ def main():
                 dts.append(d)
         value = float(np.mean(reps))
         dt = float(np.mean(dts))
+        if args.dump_outputs:  # the state the last timed sample's reverse steps ended in
+            dump_outputs(args.dump_outputs, {"angles": _CPU_TRACE["x"][-1].numpy()})
         line = {
             "impl": "reference", "metric": "backbones/sec", "value": value, "unit": "backbones/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -370,11 +396,14 @@ def main():
     noise_dev = noise_host.to(dev)
     gather = [torch.empty((B, n_pad, 6), device=dev) for _ in range(world)] if world > 1 else None
 
+    last = [None]  # the finished angles of the latest pass
+
     def one_pass_device():
         x = noise_dev.clone()
         sampling._run_steps(eng, x, start_t, wrap, None)
         if world > 1:
             dist.all_gather(gather, x)  # the job's only collective: finished angles
+        last[0] = x
         return x
 
     def barrier():
@@ -406,6 +435,8 @@ def main():
     clocks = clk.summary()
     ms_per_step = ms / args.steps
     value = world * B / (ms_per_step / 1000.0)
+    if args.dump_outputs and rank == 0:  # the finished angles of the last timed pass (all ranks' chains after the gather)
+        dump_outputs(args.dump_outputs, {"angles": (torch.cat(gather) if world > 1 else last[0]).cpu().numpy()})
 
     # ---- e2e: host noise in, host result out, through the public API ------------------------------
     e2e = None

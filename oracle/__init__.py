@@ -33,6 +33,7 @@ nerf.py       NeRF backbone builder (nerf.py:79-204), bit-identical to the refer
 writers.py    csv.gz (= the reference's own DataFrame.to_csv call) and PDB text (pinned on a reference-written file)
 loss.py       the training objective (losses.py:12-62, modelling.py:553-604, :684-685) and its gradient in closed form:
               groundwork for SURVEY 8f rank 3, no CUDA counterpart yet; bit-identical to the reference's functions
+replay.py     digests and model-call record / replay for comparing with the reference's stored answers
 ref_shims.py  sys.modules stubs that make the reference's own loop importable
               (authoring container only; /root/reference does not exist on the GPU box)
 """

@@ -1,12 +1,12 @@
 """The oracle (CPU restatement) against the golden vectors written by the reference's own code."""
 import numpy as np
-import pytest
 import torch
 
 from conftest import load_golden
 from oracle import forward as ofwd
 from oracle import loop as oloop
 from oracle import schedules as osched
+from oracle.replay import Replay, digest
 
 SEED = 7344
 
@@ -120,21 +120,36 @@ def test_chain_golden(mini_oracle):
     assert float(out.abs().max()) <= np.pi + 1e-6
 
 
-@pytest.mark.needs_reference
-def test_oracle_loop_equals_reference_loop_live(mini_oracle):
-    """Live re-check (authoring container): the reference's own loop vs the restated loop."""
-    from oracle import ref_shims
-    ref = ref_shims.load()
-    model, _, _ = mini_oracle
-    T = 20
-    betas = ref.beta_schedules.get_variance_schedule("cosine", T)
-    assert torch.equal(betas, osched.betas_for("cosine", T))
-    lens = [40, 33, 40]
+LIVE_T, LIVE_LENGTHS = 20, [40, 33, 40]
+
+
+def live_noise():
     torch.manual_seed(11)
-    noise = oloop.sample_noise(torch.zeros(3, 40, 6), [True] * 6)
+    return oloop.sample_noise(torch.zeros(3, 40, 6), [True] * 6)
+
+
+def test_oracle_loop_equals_reference_loop_live(mini_oracle):
+    """
+    The reference's own loop vs the restated loop, bit for bit.  tests/golden/ref_loop.npz holds the digest of the
+    stock p_sample_loop run around this oracle forward (tests/golden/make_golden_reference.py) and every call it made to
+    the model; the restated loop is handed the same predictions (oracle/replay.py), and the forward is checked against
+    them.
+    """
+    model, _, _ = mini_oracle
+    g = load_golden("ref_loop.npz")
+    betas = osched.betas_for("cosine", LIVE_T)
+    assert digest(betas) == str(g["loop_betas"])
+    noise = live_noise()
+    replay = Replay(g, "loop")
     torch.manual_seed(12)
-    a = ref.sampling.p_sample_loop(model, lens, noise, T, betas, is_angle=[True] * 6, disable_pbar=True)
-    torch.manual_seed(12)
-    b = oloop.p_sample_loop(model, lens, noise, T, betas, [True] * 6)
-    assert torch.equal(a, b)
-    assert torch.equal(ref.utils.modulo_with_wrapped_range(noise * 3), oloop.wrap(noise * 3))
+    b = oloop.p_sample_loop(replay, LIVE_LENGTHS, noise, LIVE_T, betas, [True] * 6)
+    assert replay.calls == replay.total == LIVE_T
+    assert digest(b) == str(g["loop_hist"])
+    assert digest(oloop.wrap(noise * 3)) == str(g["loop_wrap3"])
+    mask = torch.zeros(3, 40)
+    for i, n in enumerate(LIVE_LENGTHS):
+        mask[i, :n] = 1.0
+    for k in range(LIVE_T):  # the predictions replayed above are this forward's, to the fp32 floor of another CPU
+        x = noise if k == 0 else b[k - 1]
+        eps = model(x, torch.full((3,), LIVE_T - 1 - k), attention_mask=mask)
+        assert torch.allclose(eps, torch.from_numpy(g[f"loop_eps_{k}"]), atol=2e-6, rtol=0)

@@ -2,24 +2,17 @@
 SURVEY.md section 8f rank 3 (training step) - groundwork on the CPU: the restated objective `oracle/loss.py` pinned
 (1) on the known answers the reference's own tests hold (/root/reference/tests/test_losses.py:10-160 and the doctests of
     /root/reference/foldingdiff/losses.py:15-19, :43-44),
-(2) live and BIT-identically against the stock package in baseline/_ref: `foldingdiff.losses` and the unmodified
-    `BertForDiffusion._get_loss_terms` (modelling.py:553-604) driven with a stand-in `self`,
+(2) BIT-identically against what the stock package computed on the same inputs: `foldingdiff.losses` and the
+    unmodified `BertForDiffusion._get_loss_terms` (modelling.py:553-604) driven with a stand-in `self`,
 (3) its closed-form gradient against torch autograd through the reference's own functions.
 No CUDA kernel for this row exists yet (DESIGN.md section 0, row f); nothing here touches the product path.
 """
-import os
-import sys
-import types
-
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import load_golden
 from oracle import loss as oloss
-
-sys.path.insert(0, os.path.join(ROOT, "baseline"))
-import reference_arm  # noqa: E402
 
 IS_ANGULAR = [False, True, True, True]  # one non-angular feature, then angles (the default `is_angle` of p_sample_loop, sampling.py:84)
 IS_ANGULAR6 = [True] * 6                 # canonical-full-angles: every feature is an angle
@@ -102,69 +95,63 @@ def test_uninformed_predictor_anchor():
     assert 0.55 < got < 0.75
 
 
-# ---- (2) + (3): against the stock reference in baseline/_ref ---------------------------------------------------------
+# ---- (2) + (3): against the stock reference ------------------------------------------------------------------------
+# tests/golden/ref_loss.npz holds what the stock package (baseline/_ref) computed on these inputs: written by
+# tests/golden/make_golden_reference.py, which drives the unmodified `_get_loss_terms` with a stand-in `self`.
 
-needs_ref = pytest.mark.skipif(not reference_arm.available(), reason="baseline/_ref not installed")
+LOSS_FN_SHAPES = [(), (1,), (977,), (33, 7)]
+BETAS = (1.0, 0.1, float(torch.pi / 10))
+CIRCLE_PENALTIES = (0.0, 0.3)
+TERMS_FEATURES = [IS_ANGULAR6, IS_ANGULAR, [False, False, True]]
+GRAD_FEATURES = [IS_ANGULAR6, IS_ANGULAR]
+
+
+def loss_fn_inputs():
+    g = torch.Generator().manual_seed(11)
+    return [(20 * torch.randn(shape, generator=g), 20 * torch.randn(shape, generator=g)) for shape in LOSS_FN_SHAPES]
+
+
+def features_tag(is_angular):
+    return "".join("T" if a else "F" for a in is_angular)
 
 
 @pytest.fixture(scope="module")
 def ref():
-    _, _, _, rmodel = reference_arm.load_reference()
-    from foldingdiff import losses as rlosses  # type: ignore
-    return types.SimpleNamespace(losses=rlosses, modelling=rmodel)
+    return load_golden("ref_loss.npz")
 
 
-@needs_ref
 def test_loss_functions_bit_identical_to_the_reference(ref):
-    g = torch.Generator().manual_seed(11)
-    for shape in [(), (1,), (977,), (33, 7)]:
-        x = 20 * torch.randn(shape, generator=g)
-        y = 20 * torch.randn(shape, generator=g)
-        for beta in (1.0, 0.1, float(torch.pi / 10)):
-            for cp in (0.0, 0.3):
+    for i, (x, y) in enumerate(loss_fn_inputs()):
+        for b, beta in enumerate(BETAS):
+            for c, cp in enumerate(CIRCLE_PENALTIES):
                 ours = oloss.radian_smooth_l1(x, y, beta=beta, circle_penalty=cp)
-                theirs = ref.losses.radian_smooth_l1_loss(x, y, beta=beta, circle_penalty=cp)
-                assert torch.equal(ours, theirs), (shape, beta, cp)
-        assert torch.equal(oloss.radian_l1(x, y), ref.losses.radian_l1_loss(x, y))
+                theirs = torch.from_numpy(ref[f"fn{i}_smooth_l1_{b}_{c}"])
+                assert torch.equal(ours, theirs), (x.shape, beta, cp)
+        assert torch.equal(oloss.radian_l1(x, y), torch.from_numpy(ref[f"fn{i}_l1"]))
 
 
-def _reference_terms(ref, pred, batch, is_angular, loss="smooth_l1", circle=0.0):
-    """The unmodified `_get_loss_terms` with a stand-in `self` whose forward returns `pred`."""
-    base = ref.modelling.BertForDiffusionBase
-    fns = [base.angular_loss_fn_dict[loss] if a else base.nonangular_loss_fn_dict[loss] for a in is_angular]  # modelling.py:522-527
-    me = types.SimpleNamespace(forward=lambda *a, **k: pred, loss_func=fns, circle_lambda=circle, use_pairwise_dist_loss=0.0)
-    return ref.modelling.BertForDiffusion._get_loss_terms(me, batch)
-
-
-@needs_ref
-@pytest.mark.parametrize("is_angular", [IS_ANGULAR6, IS_ANGULAR, [False, False, True]])
+@pytest.mark.parametrize("is_angular", TERMS_FEATURES)
 @pytest.mark.parametrize("loss", ["smooth_l1", "l1"])
 def test_loss_terms_bit_identical_to_get_loss_terms(ref, is_angular, loss):
     pred, known, mask = _batch(seed=len(is_angular), F=len(is_angular))
-    batch = {"known_noise": known, "corrupted": known, "t": torch.zeros(known.shape[0], 1, dtype=torch.long),
-             "attn_mask": mask, "position_ids": torch.arange(known.shape[1])[None].expand(known.shape[0], -1)}
-    theirs = _reference_terms(ref, pred, batch, is_angular, loss)
+    theirs = torch.from_numpy(ref[f"terms_{features_tag(is_angular)}_{loss}"])
     ours = oloss.loss_terms(pred, known, mask, is_angular, loss)
     assert theirs.shape == ours.shape == (len(is_angular),)
     assert torch.equal(ours, theirs)
     assert torch.equal(oloss.training_loss(pred, known, mask, is_angular, loss), torch.mean(theirs))  # modelling.py:685
 
 
-@needs_ref
-@pytest.mark.parametrize("is_angular", [IS_ANGULAR6, IS_ANGULAR])
+@pytest.mark.parametrize("is_angular", GRAD_FEATURES)
 def test_closed_form_gradient_matches_autograd_through_the_reference(ref, is_angular):
     pred, known, mask = _batch(seed=5, F=len(is_angular))
-    pred = pred.double().requires_grad_(True)
-    known = known.double()
-    batch = {"known_noise": known, "corrupted": known, "t": None, "attn_mask": mask, "position_ids": None}
-    torch.mean(_reference_terms(ref, pred, batch, is_angular)).backward()
-    ours = oloss.training_loss_grad(pred.detach(), known, mask, is_angular)
-    assert torch.all(ours[mask == 0] == 0) and torch.all(pred.grad[mask == 0] == 0)
-    assert torch.allclose(ours, pred.grad, rtol=1e-12, atol=1e-15)
+    theirs = torch.from_numpy(ref[f"grad_{features_tag(is_angular)}"])
+    ours = oloss.training_loss_grad(pred.double(), known.double(), mask, is_angular)
+    assert torch.all(ours[mask == 0] == 0) and torch.all(theirs[mask == 0] == 0)
+    assert torch.allclose(ours, theirs, rtol=1e-12, atol=1e-15)
 
 
 def test_closed_form_gradient_matches_autograd_through_the_oracle():
-    # same check without the reference installed (the GPU box): autograd through the restatement itself
+    # the same check with autograd through the restatement itself
     for is_angular in (IS_ANGULAR6, IS_ANGULAR):
         pred, known, mask = _batch(seed=9, F=len(is_angular))
         pred = pred.double().requires_grad_(True)

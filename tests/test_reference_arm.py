@@ -1,50 +1,54 @@
-"""The reference arm of bench.py (baseline/reference_arm.py): stock reference loop + sub-modules from baseline/_ref."""
-import os
-import sys
-
-import pytest
+"""
+The reference arm of bench.py (baseline/reference_arm.py): stock reference loop + sub-modules from baseline/_ref.
+tests/golden/ref_loop.npz holds what that arm computed on the inputs below (tests/golden/make_golden_reference.py);
+the oracle must reproduce it.
+"""
 import torch
 
-from conftest import ROOT, mini_state_dict
+from conftest import load_golden, mini_state_dict
 from oracle import forward as ofwd
 from oracle import loop as oloop
 from oracle import schedules as osched
+from oracle.replay import digest
 
-sys.path.insert(0, os.path.join(ROOT, "baseline"))
-import reference_arm  # noqa: E402
-
-pytestmark = pytest.mark.skipif(not reference_arm.available(), reason="baseline/_ref not installed (see DESIGN.md section 6)")
+LOOP_T, LOOP_LENGTHS = 5, [24, 17, 24]
 
 
-def test_assembled_reference_model_matches_oracle_forward():
-    sd, cfg, _, _ = mini_state_dict()
-    model = reference_arm.build_model(sd, cfg)
-    oracle = ofwd.OracleModel(sd, ofwd.OracleConfig(**cfg), [True] * 6).eval()
+def forward_inputs():
     g = torch.Generator().manual_seed(3)
     x = torch.randn(3, 96, 6, generator=g)
     t = torch.tensor([0, 17, 249])
     mask = torch.ones(3, 96); mask[1, 60:] = 0; mask[2, 33:] = 0
+    return x, t, mask
+
+
+def loop_noise():
+    g = torch.Generator().manual_seed(11)
+    return oloop.wrap(torch.randn(3, 24, 6, generator=g))
+
+
+def test_assembled_reference_model_matches_oracle_forward():
+    sd, cfg, _, _ = mini_state_dict()
+    oracle = ofwd.OracleModel(sd, ofwd.OracleConfig(**cfg), [True] * 6).eval()
+    x, t, mask = forward_inputs()
+    got = torch.from_numpy(load_golden("ref_loop.npz")["arm_forward"])
     with torch.no_grad():
-        got, want = model(x, t, mask), oracle(x, t, attention_mask=mask)
+        want = oracle(x, t, attention_mask=mask)
     err = float((got - want)[mask.bool()].abs().max())
     print(f"reference-assembled model vs oracle forward: {err:.3e}")
     assert err < 2e-6
 
 
 def test_stock_reference_loop_drives_the_assembled_model_like_the_oracle_loop():
-    sampling, beta_schedules, _, _ = reference_arm.load_reference()
+    g = load_golden("ref_loop.npz")
     sd, cfg, _, _ = mini_state_dict()
-    model = reference_arm.build_model(sd, cfg)
     oracle = ofwd.OracleModel(sd, ofwd.OracleConfig(**cfg), [True] * 6).eval()
-    T, lengths = 5, [24, 17, 24]
-    betas = beta_schedules.get_variance_schedule("linear", T)
-    assert torch.equal(betas, osched.betas_for("linear", T))
-    g = torch.Generator().manual_seed(11)
-    noise = oloop.wrap(torch.randn(3, 24, 6, generator=g))
+    betas = osched.betas_for("linear", LOOP_T)
+    assert digest(betas) == str(g["arm_loop_betas"])
+    ref_hist = torch.from_numpy(g["arm_loop_hist"])
     torch.manual_seed(5)
-    ref_hist = sampling.p_sample_loop(model, lengths, noise.clone(), T, betas, is_angle=[True] * 6, disable_pbar=True)
-    torch.manual_seed(5)
-    ora_hist = oloop.p_sample_loop(oracle, lengths, noise.clone(), T, betas, [True] * 6)
-    worst = max(float(oloop.circular_abs_diff(ref_hist[:, i, :l], ora_hist[:, i, :l], [True] * 6).max()) for i, l in enumerate(lengths))
-    print(f"stock loop + assembled model vs oracle loop + oracle model, {T} steps: {worst:.3e}")
+    ora_hist = oloop.p_sample_loop(oracle, LOOP_LENGTHS, loop_noise(), LOOP_T, betas, [True] * 6)
+    worst = max(float(oloop.circular_abs_diff(ref_hist[:, i, :l], ora_hist[:, i, :l], [True] * 6).max())
+                for i, l in enumerate(LOOP_LENGTHS))
+    print(f"stock loop + assembled model vs oracle loop + oracle model, {LOOP_T} steps: {worst:.3e}")
     assert worst < 1e-5

@@ -53,6 +53,35 @@ def test_bench_flags_a_stale_ncu_profile(tmp_path, monkeypatch):
     assert bench.load_ncu_profile()["stale"] is True
 
 
+def test_bench_dump_outputs_writes_float32_and_a_fixed_sample_over_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    a = np.arange(40 * 3, dtype=np.float64).reshape(40, 3)
+    bench.dump_outputs(str(tmp_path / "all"), {"angles": a})
+    got = np.load(tmp_path / "all" / "angles.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, a)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 10 * 3 * 4)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"angles": a})
+    s1, s2 = (np.load(tmp_path / d / "angles.npy") for d in ("s1", "s2"))
+    assert s1.shape == (10, 3) and np.array_equal(s1, s2)  # within the limit, and the same rows every time
+    assert all(row in a.tolist() for row in s1.tolist())
+
+
+def test_bench_rejects_a_step_count_below_one(monkeypatch):
+    import pytest
+    sys.path.insert(0, ROOT)
+    import bench
+    for argv in (["--steps", "0"], ["--warmup", "-1"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse_args()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "3", "--dump-outputs", "out"])
+    args = bench.parse_args()
+    assert args.steps == 3 and args.dump_outputs == "out"
+
+
 def test_algorithmic_flops_match_survey_table():
     from foldingdiff_b200 import synthetic
     lengths = synthetic.sweep_lengths(512)
