@@ -15,7 +15,7 @@ import sys
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc")
 LIB_PATH = os.path.join(CSRC, "libfoldingdiff_b200.so")
 SOURCES = ["api.cu"]
-HEADERS = ["common.cuh", "kernels_simt.cuh", "gemm_tc.cuh", "attention_mma.cuh", "attention_pool.cuh", "attention_tc.cuh", "writers.hpp", "nerf.cuh", "philox.cuh",
+HEADERS = ["common.cuh", "kernels_simt.cuh", "gemm_tc.cuh", "attention_mma.cuh", "attention_pool.cuh", "attention_tc.cuh", "writers.hpp", "loss.cuh", "nerf.cuh", "philox.cuh",
            os.path.join("..", "..", "include", "foldingdiff_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -58,6 +58,13 @@ SIGNATURES = {
     "fd_nerf_build": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
                                   C.c_void_p, C.c_void_p]),
     "fd_randn": (C.c_int32, [C.c_void_p, C.c_int64, C.c_uint64, C.c_uint64, C.c_void_p]),
+    "fd_q_sample": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fd_loss_terms": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                  C.c_int32, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fd_pdist_loss": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                  C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                  C.c_void_p]),
     "fd_launch_count": (C.c_int64, [C.c_void_p]),
     "fd_profile_begin": (C.c_int32, [C.c_void_p]),
     "fd_profile_end": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -15,6 +15,7 @@
 #include "common.cuh"
 #include "gemm_tc.cuh"
 #include "kernels_simt.cuh"
+#include "loss.cuh"
 #include "nerf.cuh"
 #include "philox.cuh"
 
@@ -1044,6 +1045,94 @@ int32_t fd_write_batch(int32_t n_chains, const float* angles_host, int32_t n_pad
   }
   const int bad = fdw::run_batch(jobs, n_threads, gz_level);
   return bad ? fail(FD_ERR_INVALID, "%d output files could not be written", bad) : FD_OK;
+}
+
+// ---- forward half of the training step (loss.cuh; SURVEY section 8f rank 3) --------------------------------------
+int32_t fd_q_sample(const float* x0_dev, int32_t batch, int32_t n_pad, int32_t n_features, const float* sqrt_abar_dev,
+                    const float* sqrt_1m_abar_dev, const float* var_scale, const uint8_t* angular, const float* z_dev,
+                    uint64_t seed, uint64_t offset, float* known_noise_dev, float* corrupted_dev, void* stream) {
+  if (!x0_dev || !sqrt_abar_dev || !sqrt_1m_abar_dev || !var_scale || !angular || !known_noise_dev || !corrupted_dev)
+    return fail(FD_ERR_INVALID, "null argument");
+  if (batch < 1 || n_pad < 1 || n_features < 1 || n_features > FD_MAX_FEATURES)
+    return fail(FD_ERR_INVALID, "bad shape: batch=%d n_pad=%d n_features=%d", batch, n_pad, n_features);
+  fd::FeatureScales sc{};
+  uint32_t ang_bits = 0;
+  for (int f = 0; f < n_features; ++f) {
+    sc.s[f] = var_scale[f];
+    ang_bits |= (angular[f] ? 1u : 0u) << f;
+  }
+  const long long total = (long long)batch * n_pad * n_features;
+  const long long want = (total + 255) / 256;
+  fd::q_sample_kernel<<<(unsigned)(want < 4096 ? want : 4096), 256, 0, (cudaStream_t)stream>>>(
+      x0_dev, total, n_pad, n_features, sqrt_abar_dev, sqrt_1m_abar_dev, sc, ang_bits, z_dev, seed, offset,
+      known_noise_dev, corrupted_dev);
+  return check_launch();
+}
+
+int32_t fd_loss_terms(const float* eps_hat_dev, const float* known_noise_dev, const float* attn_mask_dev, int32_t batch,
+                      int32_t n_pad, int32_t n_features, const uint8_t* angular, int32_t loss, float circle_penalty,
+                      double* chain_sums_dev, float* terms_dev, void* stream) {
+  if (!eps_hat_dev || !known_noise_dev || !attn_mask_dev || !angular || !chain_sums_dev || !terms_dev)
+    return fail(FD_ERR_INVALID, "null argument");
+  if (batch < 1 || n_pad < 1 || n_features < 1 || n_features > FD_MAX_FEATURES)
+    return fail(FD_ERR_INVALID, "bad shape: batch=%d n_pad=%d n_features=%d", batch, n_pad, n_features);
+  if (loss != FD_LOSS_SMOOTH_L1 && loss != FD_LOSS_L1) return fail(FD_ERR_INVALID, "loss=%d", loss);
+  if (!(circle_penalty >= 0.0f)) return fail(FD_ERR_INVALID, "circle_penalty must be >= 0");
+  uint32_t ang_bits = 0;
+  for (int f = 0; f < n_features; ++f) ang_bits |= (angular[f] ? 1u : 0u) << f;
+  cudaStream_t st = (cudaStream_t)stream;
+  fd::loss_chain_kernel<<<batch, fd::LOSS_THREADS, 0, st>>>(eps_hat_dev, known_noise_dev, attn_mask_dev, n_pad, n_features,
+                                                             ang_bits, loss, circle_penalty > 0.0f ? 1 : 0, chain_sums_dev);
+  fd::loss_reduce_kernel<<<1, 32, 0, st>>>(chain_sums_dev, batch, n_features, circle_penalty, terms_dev);
+  return check_launch();
+}
+
+int32_t fd_pdist_loss(const float* corrupted_dev, const float* eps_hat_dev, const float* known_angles_dev,
+                      const float* sqrt_abar_dev, const float* sqrt_1m_abar_dev, const float* coef_dev, int32_t batch,
+                      int32_t n_pad, int32_t n_features, const int32_t* lengths, const int32_t* columns,
+                      float* denoised_dev, double* chain_sums_dev, float* loss_dev, void* stream) {
+  if (!corrupted_dev || !eps_hat_dev || !known_angles_dev || !sqrt_abar_dev || !sqrt_1m_abar_dev || !coef_dev || !lengths ||
+      !columns || !loss_dev)
+    return fail(FD_ERR_INVALID, "null argument");
+  if (batch < 1 || n_pad < 1 || n_pad > 128 || n_features < 3 || n_features > FD_MAX_FEATURES)
+    return fail(FD_ERR_INVALID, "bad shape: batch=%d n_pad=%d (<= 128) n_features=%d", batch, n_pad, n_features);
+  for (int i = 0; i < 6; ++i)
+    if (columns[i] >= n_features || (i < 3 && columns[i] < 0))
+      return fail(FD_ERR_INVALID, "columns[%d]=%d (phi, psi, omega are required; all must be < n_features)", i, columns[i]);
+  for (int b = 0; b < batch; ++b)
+    if (lengths[b] < 1 || lengths[b] > n_pad) return fail(FD_ERR_INVALID, "lengths[%d]=%d outside [1, %d]", b, lengths[b], n_pad);
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t n_ang = (size_t)batch * n_pad * n_features, n_xyz = (size_t)batch * n_pad * 9;
+  // stream-ordered scratch: freed behind the kernels, so the call does not synchronise
+  char* work = nullptr;
+  const size_t bytes = sizeof(float) * (2 * n_xyz + (denoised_dev ? 0 : n_ang)) + sizeof(double) * (chain_sums_dev ? 0 : 2 * (size_t)batch) +
+                       sizeof(int) * (size_t)batch + 64;
+  FD_CUDA(cudaMallocAsync((void**)&work, bytes, st));
+  float* xyz_a = (float*)work;
+  float* xyz_b = xyz_a + n_xyz;
+  float* den = denoised_dev ? denoised_dev : xyz_b + n_xyz;
+  char* tail = (char*)(denoised_dev ? xyz_b + n_xyz : den + n_ang);
+  tail = (char*)(((uintptr_t)tail + 15) & ~(uintptr_t)15);
+  double* chain = chain_sums_dev ? chain_sums_dev : (double*)tail;
+  int* d_len = (int*)(chain_sums_dev ? tail : tail + sizeof(double) * 2 * (size_t)batch);
+  int rc = FD_OK;
+  if (cudaMemcpyAsync(d_len, lengths, sizeof(int) * batch, cudaMemcpyHostToDevice, st) != cudaSuccess)
+    rc = fail(FD_ERR_CUDA, "pdist: H2D lengths");
+  if (!rc) {
+    const long long total = (long long)n_ang, want = (total + 255) / 256;
+    fd::denoise_kernel<<<(unsigned)(want < 4096 ? want : 4096), 256, 0, st>>>(corrupted_dev, eps_hat_dev, total,
+                                                                              (long long)n_pad * n_features, sqrt_abar_dev,
+                                                                              sqrt_1m_abar_dev, den);
+    // both structures through the library's one NeRF (nerf.cuh), uncentred: the term is translation invariant
+    const fd::NerfCols cols{columns[0], columns[1], columns[2], columns[3], columns[4], columns[5]};
+    fd::nerf_kernel<<<(batch + 31) / 32, 32, 0, st>>>(den, d_len, batch, n_pad, n_features, cols, 0, xyz_a);
+    fd::nerf_kernel<<<(batch + 31) / 32, 32, 0, st>>>(known_angles_dev, d_len, batch, n_pad, n_features, cols, 0, xyz_b);
+    fd::pdist_chain_kernel<<<batch, fd::LOSS_THREADS, 0, st>>>(xyz_a, xyz_b, d_len, n_pad, coef_dev, chain);
+    fd::pdist_reduce_kernel<<<1, 32, 0, st>>>(chain, batch, loss_dev);
+    rc = check_launch();
+  }
+  cudaFreeAsync(work, st);
+  return rc;
 }
 
 int32_t fd_debug_tc_status(void) { return fd::tc_check_error(); }

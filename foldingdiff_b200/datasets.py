@@ -195,4 +195,112 @@ class SyntheticAnglesDataset:
                 "position_ids": torch.arange(self.pad)}
 
 
+class AnglesTableDataset:
+    """
+    Held-out structures given as angle tables, producing the item of the reference's CathCanonicalAnglesOnlyDataset
+    (datasets.py:364-460): "angles" (pad, F) fp32, "attn_mask", "position_ids", "lengths".  Wrap it in
+    NoisedAnglesDataset to evaluate a model's loss (losses.validation_loss).
+
+    `tables` is a directory of the *.csv.gz angle tables bin/sample.py / writers.py write (read in sorted file-name
+    order, pandas index_col=0, feature-name header), or a sequence of (L, F) arrays / DataFrames in the model's feature
+    order.  Per item, as the reference does:
+      * subtract `mean_offset` (the model dir's training_mean_offset.npy) and wrap the angular columns to [-pi, pi)
+      * NaN -> 0
+      * pad to `pad`, or trim longer tables by `trim_strategy`: "leftalign" keeps the first `pad` rows, "randomcrop"
+        a window drawn from np.random.default_rng(6489), "discard" drops such tables at load (datasets.py:175-183)
+    """
+
+    def __init__(self, tables, feature_set_key: str = "canonical-full-angles", pad: int = 128,
+                 mean_offset: Optional[np.ndarray] = None, trim_strategy: str = "leftalign"):
+        if trim_strategy not in ("leftalign", "randomcrop", "discard"):
+            raise ValueError(f"Unknown trim strategy: {trim_strategy}")
+        key = "coords" if feature_set_key == "cart-coords" else "angles"
+        self.feature_is_angular = {key: FEATURE_SET_NAMES_TO_ANGULARITY[feature_set_key]}
+        self.feature_names = {key: FEATURE_SET_NAMES_TO_FEATURE_NAMES[feature_set_key]}
+        self._key = key
+        self.pad = pad
+        self.trim_strategy = trim_strategy
+        self.rng = np.random.default_rng(seed=6489)  # datasets.py:111
+        self._mean_offset = None if mean_offset is None else np.asarray(mean_offset, dtype=np.float64)
+        names = self.feature_names[key]
+        if self._mean_offset is not None:
+            assert self._mean_offset.size == len(names), f"mean offset has {self._mean_offset.size} entries"
+        if isinstance(tables, (str, os.PathLike)):
+            import glob
+            paths = sorted(glob.glob(os.path.join(os.fspath(tables), "*.csv.gz")))
+            if not paths:
+                raise FileNotFoundError(f"no *.csv.gz angle tables in {tables}")
+            arrays, self.filenames = [], []
+            for p in paths:
+                arrays.append(self._read_table(p, names))
+                self.filenames.append(p)
+        else:
+            arrays = [self._as_array(t, names) for t in tables]
+            self.filenames = [f"table_{i}" for i in range(len(arrays))]
+        if trim_strategy == "discard":
+            keep = [i for i, a in enumerate(arrays) if a.shape[0] <= pad]
+            logging.info(f"Removing structures longer than {pad} keeps {len(keep)}/{len(arrays)}")
+            arrays = [arrays[i] for i in keep]
+            self.filenames = [self.filenames[i] for i in keep]
+        self._tables = arrays
+
+    @staticmethod
+    def _read_table(path: str, names) -> np.ndarray:
+        import pandas as pd
+        df = pd.read_csv(path, index_col=0)
+        missing = [n for n in names if n not in df.columns]
+        if missing:
+            raise ValueError(f"{path}: missing feature columns {missing}")
+        return df.loc[:, names].to_numpy(dtype=np.float64)
+
+    @staticmethod
+    def _as_array(t, names) -> np.ndarray:
+        if hasattr(t, "loc") and hasattr(t, "columns"):
+            return t.loc[:, names].to_numpy(dtype=np.float64)
+        a = np.asarray(t, dtype=np.float64)
+        if a.ndim != 2 or a.shape[1] != len(names):
+            raise ValueError(f"expected an (L, {len(names)}) table, got {a.shape}")
+        return a
+
+    @classmethod
+    def from_model_dir(cls, tables, model_dir: str) -> "AnglesTableDataset":
+        """Feature set, pad, trim strategy and mean offset of a training output directory."""
+        with open(os.path.join(model_dir, "training_args.json")) as f:
+            targs = json.load(f)
+        offset_file = os.path.join(model_dir, "training_mean_offset.npy")
+        offset = np.load(offset_file) if os.path.isfile(offset_file) else None
+        return cls(tables, targs["angles_definitions"], pad=targs["max_seq_len"], mean_offset=offset,
+                   trim_strategy=targs.get("trim_strategy", "leftalign"))
+
+    def get_masked_means(self):
+        return None if self._mean_offset is None else np.copy(self._mean_offset)
+
+    def __len__(self) -> int:
+        return len(self._tables)
+
+    def __getitem__(self, index, ignore_zero_center: bool = False) -> Dict[str, torch.Tensor]:
+        if not 0 <= index < len(self):
+            raise IndexError("Index out of range")
+        angles = self._tables[index].copy()
+        if self._mean_offset is not None and not ignore_zero_center:
+            angles = angles - self._mean_offset
+            idx = np.where(self.feature_is_angular[self._key])[0]
+            angles[:, idx] = utils.modulo_with_wrapped_range(angles[:, idx], -np.pi, np.pi)
+        np.nan_to_num(angles, copy=False, nan=0)
+        l = min(self.pad, angles.shape[0])
+        attn_mask = torch.zeros(size=(self.pad,))
+        attn_mask[:l] = 1.0
+        if angles.shape[0] < self.pad:
+            angles = np.pad(angles, ((0, self.pad - angles.shape[0]), (0, 0)), mode="constant", constant_values=0)
+        elif angles.shape[0] > self.pad:
+            if self.trim_strategy == "randomcrop":
+                start = self.rng.integers(0, angles.shape[0] - self.pad)
+                angles = angles[start:start + self.pad]
+            else:
+                angles = angles[: self.pad]
+        return {self._key: torch.from_numpy(np.ascontiguousarray(angles)).float(), "attn_mask": attn_mask,
+                "position_ids": torch.arange(start=0, end=self.pad, step=1, dtype=torch.long),
+                "lengths": torch.tensor(l, dtype=torch.int64)}
+
+
 logging.getLogger(__name__).addHandler(logging.NullHandler())

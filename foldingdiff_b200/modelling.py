@@ -8,7 +8,8 @@ Drop-in for the parts of /root/reference/foldingdiff/modelling.py that the sampl
   * `.to(device) / .eval() / .parameters() / .state_dict()`, `.n_inputs`, `.ft_is_angular`,
     `.ft_names`, `.config`
   * `BertForDiffusion` - in the reference a pytorch-lightning training wrapper (:487-804); here
-    the same loader/forward (training is out of scope).
+    the same loader/forward plus the evaluation half of training: the reference's constructor kwargs,
+    `_get_loss_terms` and `validation_step` on the device (the backward pass is out of scope).
 
 What is different by design: there is no HuggingFace `BertEncoder` and no PyTorch eager forward.
 The module only *holds* the parameters under the reference's state-dict names (so checkpoints
@@ -24,12 +25,12 @@ import os
 import re
 import shutil
 from pathlib import Path
-from typing import List, Literal, Optional, Sequence
+from typing import Dict, List, Literal, Optional, Sequence, Union
 
 import torch
 from torch import nn
 
-from . import _native, engine
+from . import _native, engine, losses
 from .datasets import FEATURE_SET_NAMES_TO_ANGULARITY
 
 TIME_ENCODING = Literal["gaussian_fourier", "sinusoidal"]
@@ -69,6 +70,20 @@ class _Holder(nn.Module):
 
 def _linear(i: int, o: int) -> nn.Linear:
     return nn.Linear(i, o)
+
+
+def mask_layout(attention_mask: torch.Tensor):
+    """
+    -> (lengths, mask_cpu, is_prefix) of a (B, N) attention mask: per-chain valid-token counts, the mask as fp32 on the
+    host, and whether every row is a prefix mask (tokens [0, lengths[b]) valid, lengths[b] >= 1) - the layout the
+    packed-row path of fd_set_batch serves without a key mask.
+    """
+    mask_cpu = attention_mask.detach().to("cpu", torch.float32)
+    N = mask_cpu.shape[1]
+    lengths = mask_cpu.sum(dim=1).to(torch.int64)
+    prefix = torch.arange(N)[None, :] < lengths[:, None]
+    is_prefix = bool(torch.equal(prefix, mask_cpu > 0.5)) and bool((lengths >= 1).all())
+    return lengths.tolist(), mask_cpu, is_prefix
 
 
 class BertForDiffusionBase(nn.Module):
@@ -235,12 +250,9 @@ class BertForDiffusionBase(nn.Module):
         assert inputs.dim() == 3
         eng = self.native_engine()
         B, N, _ = inputs.shape
-        mask_cpu = attention_mask.detach().to("cpu", torch.float32)
-        lengths = mask_cpu.sum(dim=1).to(torch.int64)
-        prefix = torch.arange(N)[None, :] < lengths[:, None]
-        is_prefix = bool(torch.equal(prefix, mask_cpu > 0.5)) and bool((lengths >= 1).all())
+        lengths, mask_cpu, is_prefix = mask_layout(attention_mask)
         if is_prefix:
-            eng.set_batch(lengths.tolist(), N, all_rows=True)
+            eng.set_batch(lengths, N, all_rows=True)
         else:
             eng.set_batch([N] * B, N, all_rows=True, key_mask=mask_cpu)
         t = timestep.detach().reshape(-1).to("cpu")
@@ -250,4 +262,100 @@ class BertForDiffusionBase(nn.Module):
 
 
 class BertForDiffusion(BertForDiffusionBase):
-    """Name kept for `BertForDiffusion.from_dir(...)` call sites (README.md:55-77 of the reference)."""
+    """
+    The reference's training wrapper (modelling.py:487-804) as far as evaluation goes: it takes the training kwargs of
+    bin/train.py:446-459 and evaluates the training objective on the device (`_get_loss_terms`, `validation_step`;
+    kernels in csrc/loss.cuh).  The backward pass, the optimizer and dropout are not implemented: `training_step` raises.
+    `lr`, `l1`, `l2`, `epochs`, `steps_per_epoch` and `lr_scheduler` are stored for signature compatibility only.
+    """
+
+    def __init__(self, lr: float = 5e-5, loss: str = "smooth_l1",
+                 use_pairwise_dist_loss: Union[float, Sequence[float]] = 0.0, l2: float = 0.0, l1: float = 0.0,
+                 circle_reg: float = 0.0, epochs: int = 1, steps_per_epoch: int = 250, lr_scheduler=None,
+                 write_preds_to_dir: Optional[str] = None, **kwargs):
+        super().__init__(**kwargs)
+        if callable(loss) or not isinstance(loss, str):
+            raise NotImplementedError(f"loss={loss!r}: only the named losses {sorted(losses.LOSS_KINDS)} (and the "
+                                      "autocorrected 'radian_l1_smooth') have device kernels; a callable loss does not")
+        loss = losses.LOSS_AUTOCORRECT.get(loss, loss)  # modelling.py:515-521
+        if loss not in losses.LOSS_KINDS:
+            raise ValueError(f"loss={loss!r}: expected one of {sorted(losses.LOSS_KINDS)} or 'radian_l1_smooth'")
+        if write_preds_to_dir:
+            raise NotImplementedError("write_preds_to_dir: writing validation predictions is not implemented")
+        self.loss = loss
+        self.learning_rate = lr
+        self.use_pairwise_dist_loss = list(use_pairwise_dist_loss) if isinstance(use_pairwise_dist_loss, (list, tuple)) \
+            else float(use_pairwise_dist_loss)
+        self.l1_lambda, self.l2_lambda = l1, l2
+        self.circle_lambda = float(circle_reg)
+        self.epochs, self.steps_per_epoch, self.lr_scheduler = epochs, steps_per_epoch, lr_scheduler
+        self.write_preds_to_dir = None
+
+    @property
+    def pdist_enabled(self) -> bool:
+        """modelling.py:610-613: the list form, or a positive scalar, switches the pairwise-distance term on."""
+        return isinstance(self.use_pairwise_dist_loss, list) or self.use_pairwise_dist_loss > 0
+
+    def _circle_mask(self) -> torch.Tensor:
+        """1.0 for the features whose loss carries the circle penalty (angular smooth-L1), else 0.0."""
+        on = self.loss == "smooth_l1" and self.circle_lambda > 0
+        return torch.tensor([1.0 if (a and on) else 0.0 for a in self.ft_is_angular], dtype=torch.float64)
+
+    @torch.no_grad()
+    def _loss_terms_detail(self, batch):
+        """_get_loss_terms plus the per-chain sums the terms were reduced from (validation_loss builds its per-timestep
+        table from them): -> (terms, {"eps_hat", "chain_sums"[, "pdist_chain_sums"]})."""
+        eng = self.native_engine()
+        dev = next(self.parameters()).device
+        corrupted = batch["corrupted"].detach().to(dev, torch.float32).contiguous()
+        known = batch["known_noise"].detach().to(dev, torch.float32).contiguous()
+        assert corrupted.dim() == 3 and known.shape == corrupted.shape, f"{known.shape} != {corrupted.shape}"
+        attn_mask = batch["attn_mask"]
+        assert attn_mask.dim() == 2
+        B, N, _ = corrupted.shape
+        lengths, mask_cpu, is_prefix = mask_layout(attn_mask)
+        pdist_lengths = None
+        if self.pdist_enabled:
+            pdist_lengths = [int(l) for l in batch["lengths"].reshape(-1).tolist()]
+        # Only the rows the loss reads are computed: padded rows enter no term (the pairwise term reads rows below
+        # batch["lengths"], which a dataset item sets to the mask's length).
+        if is_prefix and (pdist_lengths is None or all(p <= l for p, l in zip(pdist_lengths, lengths))):
+            eng.set_batch(lengths, N, all_rows=False)
+        else:
+            eng.set_batch([N] * B, N, all_rows=True, key_mask=mask_cpu)
+        t = batch["t"].detach().reshape(-1).to("cpu")
+        temb = self._time_rows(t).to(dev)
+        eps_hat = eng.forward(corrupted, temb)
+        terms, chain = losses.loss_terms(eps_hat, known, attn_mask.to(dev), self.ft_is_angular, self.loss,
+                                         self.circle_lambda)
+        detail = {"eps_hat": eps_hat, "chain_sums": chain}
+        if self.pdist_enabled:
+            tt = batch["t"].detach().to(dev)
+            coef = losses.pdist_coefficients(self.use_pairwise_dist_loss, tt)
+            pd, pchain = losses.pdist_loss(corrupted, eps_hat, batch["angles"].to(dev),
+                                           batch["sqrt_alphas_cumprod_t"].to(dev),
+                                           batch["sqrt_one_minus_alphas_cumprod_t"].to(dev), coef, pdist_lengths,
+                                           self.ft_names)
+            terms = torch.cat([terms, pd.reshape(1)])
+            detail["pdist_chain_sums"] = pchain
+        return terms, detail
+
+    def _get_loss_terms(self, batch, write_preds: Optional[str] = None) -> torch.Tensor:
+        """
+        The reference's _get_loss_terms (modelling.py:553-677) on the device: (F,) per-feature terms, (F+1,) with the
+        pairwise-distance term, fp32 on the model's device.  `batch` is the default_collate of NoisedAnglesDataset
+        items (corrupted, t, known_noise, attn_mask, position_ids, lengths, angles, sqrt_*_t), on CPU or CUDA.
+        The network runs on the valid rows only when the mask is a prefix mask (exact: padded rows enter no term).
+        """
+        if write_preds is not None:
+            raise NotImplementedError("write_preds: writing validation predictions is not implemented")
+        return self._loss_terms_detail(batch)[0]
+
+    def validation_step(self, batch, batch_idx) -> Dict[str, torch.Tensor]:
+        """modelling.py:719-750, without the logging: {"val_loss": mean of the terms}."""
+        return {"val_loss": torch.mean(self._get_loss_terms(batch))}
+
+    def training_step(self, batch, batch_idx):
+        raise NotImplementedError("training_step needs the backward pass (gradient of the loss through the network) and "
+                                  "the optimizer, which foldingdiff_b200 does not implement; evaluate with "
+                                  "_get_loss_terms / validation_step / losses.validation_loss")

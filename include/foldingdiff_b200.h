@@ -237,6 +237,62 @@ int32_t fd_nerf_build(const float* angles_dev, int32_t batch, int32_t n_pad, int
                       const int32_t* lengths, const int32_t* columns, int32_t center, float* coords_out_dev,
                       void* stream);
 
+/* ---- forward half of the training step (SURVEY.md section 8f, rank 3) ------------------------------------------
+ * Device pointers, fp32 unless stated, work enqueued on `stream`, no synchronisation; bad shapes / arguments return
+ * FD_ERR_INVALID.  Together with fd_forward they evaluate BertForDiffusion._get_loss_terms
+ * (/root/reference/foldingdiff/modelling.py:553-677) on the device.
+ *
+ * fd_q_sample <- NoisedAnglesDataset.sample_noise + __getitem__ (/root/reference/foldingdiff/datasets.py:772-799,
+ *   :801-886), for a whole batch:
+ *     known_noise = scale_f * z,                              wrapped into [-pi, pi) where angular[f]
+ *     corrupted   = sqrt_abar_b * x0 + sqrt_1m_abar_b * known_noise,   wrapped where angular[f]
+ *   in torch's fp32 op order, bit-identical to the host mirror given the same z.
+ *     x0_dev (batch, n_pad, F); sqrt_abar_dev / sqrt_1m_abar_dev (batch); var_scale HOST float[F]; angular HOST
+ *     uint8[F]; z_dev (batch, n_pad, F) standard normals, or NULL: element i = (b * n_pad + n) * F + f then is element
+ *     offset + i of the library's Philox stream `seed` (what fd_randn(seed, offset) writes at index i).
+ */
+int32_t fd_q_sample(const float* x0_dev, int32_t batch, int32_t n_pad, int32_t n_features, const float* sqrt_abar_dev,
+                    const float* sqrt_1m_abar_dev, const float* var_scale, const uint8_t* angular, const float* z_dev,
+                    uint64_t seed, uint64_t offset, float* known_noise_dev, float* corrupted_dev, void* stream);
+
+/* Loss kinds of fd_loss_terms (BertForDiffusion's `loss` argument, modelling.py:224-237). */
+enum {
+  FD_LOSS_SMOOTH_L1 = 0, /* angular: radian_smooth_l1_loss, beta = pi/10; other: F.smooth_l1_loss (beta = 1) */
+  FD_LOSS_L1 = 1         /* angular: radian_l1_loss;                       other: F.l1_loss                  */
+};
+
+/*
+ * fd_loss_terms <- the per-feature loop of _get_loss_terms (modelling.py:571-604, losses.py:12-62): terms_dev[f] =
+ * mean over the tokens with attn_mask != 0 of the feature-f loss between eps_hat and known_noise, plus
+ * circle_penalty * mean(trunc(|eps_hat| / pi)) on angular features when loss == FD_LOSS_SMOOTH_L1.
+ *   eps_hat_dev, known_noise_dev (batch, n_pad, F); attn_mask_dev (batch, n_pad); angular HOST uint8[F]
+ *   chain_sums_dev (batch, 2F + 1) fp64, written: per chain the loss sums of each feature, the circle sums of each
+ *                  feature and the valid-token count (what a per-timestep table is built from)
+ *   terms_dev      (F), written
+ * Every sum is taken in one fixed order in fp64 (no atomics): two runs give the same bits.
+ */
+int32_t fd_loss_terms(const float* eps_hat_dev, const float* known_noise_dev, const float* attn_mask_dev, int32_t batch,
+                      int32_t n_pad, int32_t n_features, const uint8_t* angular, int32_t loss, float circle_penalty,
+                      double* chain_sums_dev, float* terms_dev, void* stream);
+
+/*
+ * fd_pdist_loss <- the pairwise-distance branch of _get_loss_terms (modelling.py:616-677, losses.py:66-150):
+ *   denoised = (corrupted - sqrt_1m_abar_b * eps_hat) / sqrt_abar_b   (not wrapped, the reference's fp32 op order)
+ *   both denoised and known_angles go through the NeRF of fd_nerf_build (uncentred); over the CA atoms of chain b,
+ *   pairs i < j < lengths[b]:  loss = sum_b coef_b * sum (|a_i - a_j| - |k_i - k_j|)^2 / (number of pairs in the batch)
+ *   known_angles_dev is the batch's "angles": the reference builds the known structure from the zero-centred angles.
+ *   corrupted_dev, eps_hat_dev, known_angles_dev (batch, n_pad, F); sqrt_* and coef_dev (batch) fp32
+ *   lengths HOST int32[batch] in [1, n_pad]; columns HOST int32[6] as for fd_nerf_build; n_pad <= 128
+ *   denoised_dev   (batch, n_pad, F) written, or NULL
+ *   chain_sums_dev (batch, 2) fp64 written (weighted squared-difference sum, pair count), or NULL
+ *   loss_dev       (1) written
+ * Scratch is stream-ordered (cudaMallocAsync / cudaFreeAsync); distances and sums in fp64, fixed order.
+ */
+int32_t fd_pdist_loss(const float* corrupted_dev, const float* eps_hat_dev, const float* known_angles_dev,
+                      const float* sqrt_abar_dev, const float* sqrt_1m_abar_dev, const float* coef_dev, int32_t batch,
+                      int32_t n_pad, int32_t n_features, const int32_t* lengths, const int32_t* columns,
+                      float* denoised_dev, double* chain_sums_dev, float* loss_dev, void* stream);
+
 /* Fill dst_dev[0..n) with standard normals from the library's Philox4x32-10 stream
  * (seed, offset).  Used by fd_sample_host(noise_host == NULL) and the throughput mode. */
 int32_t fd_randn(float* dst_dev, int64_t n, uint64_t seed, uint64_t offset, void* stream);
